@@ -64,7 +64,32 @@ def parse():
     ap.add_argument("--no-api-leg", action="store_true", help="e2e through the C ABI only (skips the Henbun-API leg)")
     ap.add_argument("--engine", type=int, default=0, help="GEMM engine: 0 auto, 1 SIMT fp32, 2 tcgen05 3xTF32")
     ap.add_argument("--profile-csv", default=None, help="dump the per-launch GEMM events of the profiled step to this file")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step computed as DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs needs --impl ours (the reference arm draws other samples at another N)")
+    return a
+
+
+DUMP_BYTES = 60 << 20          # all files of --dump-outputs together, .npy headers included, stay under 64 MB
+
+
+def dump_outputs(path, arrays):
+    """Write each tensor of `arrays` ({name: fp32 or fp64 tensor}) as path/<name>.npy.  A tensor larger than its equal share of
+    DUMP_BYTES is written as a sample of its flattened elements at seeded positions, the same in every run, so that the
+    files of two builds compare element for element."""
+    import torch
+    os.makedirs(path, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, t in arrays.items():
+        t = torch.as_tensor(t).detach()
+        if t.numel() * t.element_size() > share:
+            idx = np.unique(np.random.default_rng(0).integers(0, t.numel(), share // t.element_size()))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.cpu().numpy())
 
 
 def extrapolation_factor(n_full, n_sample, S):
@@ -105,7 +130,7 @@ class ClockSampler:
          "clocks_event_reasons.sw_power_cap")
 
     def __init__(self, gpu_index):
-        self.f = tempfile.NamedTemporaryFile("w+", suffix=".csv", delete=False)
+        self.f = tempfile.TemporaryFile("w+")
         self.idx = gpu_index
         self.p = None
 
@@ -219,16 +244,8 @@ class Dist:
 
 
 def peaks():
-    p = {}
-    try:
-        p = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
-    except Exception:
-        pass
-    tf = p.get("bf16_tflops_sustained"); hbm = p.get("hbm_gbs")
-    src = "measured (MEASURED_PEAKS.json: bf16 dense sustained / HBM copy)"
-    if tf is None or hbm is None:
-        tf, hbm, src = tf or 1400.0, hbm or 6500.0, "fallback (B200_PROFILING.md)"
-    return tf, hbm, src
+    """The ceilings the rooflines divide by: bf16 dense sustained TFLOP/s and HBM copy GB/s (BASELINE.md section 2)."""
+    return 1415.5, 6550.0, "measured on one B200 at its 1,000 W power limit: bf16 dense sustained / HBM copy (BASELINE.md section 2)"
 
 
 def ncu_traffic():
@@ -390,9 +407,13 @@ def run_c3(d, a):
     if d.rank == 0:
         clocks.start()
     l0 = lib.hb_launch_count()
-    ms = d.timed(lambda i: g.step(), a.steps)
+    try:
+        ms = d.timed(lambda i: g.step(), a.steps)
+    finally:                                   # the nvidia-smi sampler must not outlive a failing step
+        clk = clocks.stop() if d.rank == 0 else None
     launches = lib.hb_launch_count() - l0
-    clk = clocks.stop() if d.rank == 0 else None
+    if a.dump_outputs and d.rank == 0:         # out4 = {ELBO, loglik_sum, kl_sum, 0}; params after the step's Adam update
+        dump_outputs(a.dump_outputs, {"out4": g.out4, "grads": g.grads, "params": g.params})
     ms_cabi_e2e = d.timed(lambda i: g.step(host_io=True), min(a.steps, 3)) / min(a.steps, 3)
     # separate, untimed passes for the evidence: per-launch GEMM events (roofline) and per-phase events
     d.barrier()
@@ -613,7 +634,7 @@ def run_c1(d, steps=200):
             "elbo_last": float(out4[0]), "err_flag": int(err.item())}
 
 
-def run_c5(d, steps, warmup, S=64, M=65536, n=16384):
+def run_c5(d, steps, warmup, dump=None, S=64, M=65536, n=16384):
     """Config 5: full-covariance q over n = 16384 latents seen through a dense 65536 x 16384 operator; the operator is
     row-sharded over the ranks (strong scaling in M), one all-reduce of [S n + 4] floats per step."""
     import torch
@@ -639,6 +660,8 @@ def run_c5(d, steps, warmup, S=64, M=65536, n=16384):
     for _ in range(warmup):
         step(False)
     ms = d.timed(lambda i: step(False), steps) / steps
+    if dump and d.rank == 0:
+        dump_outputs(dump, {"out4": st.out4, "q_mu": st.q_mu, "q_sqrt": st.q_sqrt, "var_free": st.var_free})
     ms_e2e = d.timed(lambda i: step(True), steps) / steps
     tri = n * (n + 1) / 2
     bytes_step = 2 * 4.0 * rows * n + 4 * tri + 4.0 * S * (3 * rows + 4 * n) + 6 * 4 * tri + 4.0 * S * n * 4
@@ -657,7 +680,7 @@ def run_c5(d, steps, warmup, S=64, M=65536, n=16384):
     return out
 
 
-def run_c4(d, steps, warmup, n_data=1000000, B=4096, S=32, latent=64):
+def run_c4(d, steps, warmup, dump=None, n_data=1000000, B=4096, S=32, latent=64):
     """Config 4: amortised encoder 784-512-512-2x64 + mirrored decoder, 1 M synthetic points resident in HBM, minibatch
     4096 (split over the ranks), S = 32, through the Henbun API."""
     import torch
@@ -694,6 +717,8 @@ def run_c4(d, steps, warmup, n_data=1000000, B=4096, S=32, latent=64):
     for _ in range(warmup):
         step(False)
     ms = d.timed(lambda i: step(False), steps) / steps
+    if dump and d.rank == 0:                   # the objective optimize() returned and the flat parameter vector it updated
+        dump_outputs(dump, {"elbo": opt.last_objective, "params": opt._flat})
     ms_e2e = d.timed(lambda i: step(True), steps) / steps
     flop = 3 * 2.0 * B * (784 * 512 + 512 * 512 + 512 * 2 * latent) + 3 * 2.0 * B * S * (latent * 512 + 512 * 512 + 512 * 784)
     tf_peak, _h, src = peaks()
@@ -759,7 +784,7 @@ def measure(a):
             if line is not None:
                 line["other_workloads"] = extras
     else:
-        r = run_c5(d, a.steps, a.warmup) if a.workload == "c5" else run_c4(d, a.steps, a.warmup)
+        r = (run_c5 if a.workload == "c5" else run_c4)(d, a.steps, a.warmup, a.dump_outputs)
         if d.rank == 0:
             line = {"metric": METRIC, "value": r["value"], "unit": UNIT, "n_gpus": d.world, "steps": a.steps, "warmup": a.warmup,
                     "ms_per_step": r["ms_per_step"], "higher_is_better": True, "scaling": "strong", "vs_baseline": None, "dtype": "f32",

@@ -1,8 +1,8 @@
 #!/usr/bin/env python
-"""Generate tests/golden/*.npz by executing the UNMODIFIED reference (/root/reference/Henbun) on the
+"""Generate tests/golden/*.npz by executing the UNMODIFIED reference (a checkout of fujii-team/Henbun) on the
 TF-1 shim of tests/golden/tf1_shim.py (TensorFlow itself is not installable here).
 
-    python tests/golden/make_golden.py          # needs /root/reference; the GPU box never runs this
+    HENBUN_REFERENCE=<checkout of fujii-team/Henbun> python tests/golden/make_golden.py
 
 Every vector below is produced by the reference's own Python: its Variational sampler / KL, kernels,
 Cholesky wrapper, NeuralNet, LOCAL feed routing, densities, transforms, the notebook models' ELBO,
@@ -20,7 +20,7 @@ sys.path.insert(0, HERE)
 import tf1_shim  # noqa: E402
 
 tf = tf1_shim.install()
-sys.path.insert(0, "/root/reference")
+sys.path.insert(0, os.environ["HENBUN_REFERENCE"])
 warnings.simplefilter("ignore")
 import Henbun as hb  # noqa: E402  (the reference)
 

@@ -3,7 +3,7 @@
 Purpose: TensorFlow cannot be installed in this image, but the reference (fujii-team/Henbun) is pure
 Python on top of ~60 TF-1 symbols.  This shim provides exactly those symbols so that
 ``tests/golden/make_golden.py`` can import and execute the UNMODIFIED reference modules from
-/root/reference and record what the reference's own code computes (sampler, KL, kernels, Cholesky,
+a checkout of it and record what the reference's own code computes (sampler, KL, kernels, Cholesky,
 NeuralNet, LOCAL feed, ELBO of the notebook models, tf.gradients of all of it, AdamOptimizer steps).
 The recorded vectors are committed under tests/golden/*.npz and pin the oracle.
 

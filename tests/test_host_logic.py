@@ -171,6 +171,23 @@ def test_bench_cpu_extrapolation_rule():
     assert bench.host_threads() >= 1
 
 
+def test_bench_dump_outputs_cap_and_fixed_sample(tmp_path, monkeypatch):
+    import importlib.util, os
+    spec = importlib.util.spec_from_file_location("bench", os.path.join(os.path.dirname(os.path.dirname(__file__)), "bench.py"))
+    bench = importlib.util.module_from_spec(spec); spec.loader.exec_module(bench)
+    assert bench.DUMP_BYTES + 4096 < 64e6
+    monkeypatch.setattr(bench, "DUMP_BYTES", 8192)                                   # shares of 4 KB: "big" is sampled
+    big = torch.arange(100000, dtype=torch.float32).reshape(250, 400)
+    small = torch.tensor([[1.0, 2.0]], dtype=torch.float64)
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), {"big": big, "small": small})
+    a, b = np.load(tmp_path / "a" / "big.npy"), np.load(tmp_path / "b" / "big.npy")
+    assert a.dtype == np.float32 and 0 < a.nbytes <= 4096 and np.array_equal(a, b)    # same positions in every run
+    assert np.all(np.diff(a) > 0) and a[-1] < 100000                                  # distinct elements of the array
+    s = np.load(tmp_path / "a" / "small.npy")
+    assert s.dtype == np.float64 and s.shape == (1, 2) and np.array_equal(s, [[1.0, 2.0]])
+
+
 def test_philox4x32_10_published_algorithm_reproduces_the_kat_vectors():
     """Independent restatement of Philox-4x32-10 (Salmon et al. 2011: multipliers 0xD2511F53 / 0xCD9E8D57, Weyl key
     increments 0x9E3779B9 / 0xBB67AE85) against the three Random123 known-answer vectors that the GPU test

@@ -208,14 +208,15 @@ def test_expert_gpr_model():
 
 
 def test_golden_vectors_regenerate_from_the_reference(tmp_path):
-    """The committed vectors are exactly what the UNMODIFIED reference (/root/reference, on the TF-1 shim) produces:
-    re-run the generator into a scratch directory and compare array by array.  Skipped where the reference tree is
-    absent (the GPU box)."""
+    """The committed vectors are exactly what the UNMODIFIED reference (the checkout of fujii-team/Henbun that
+    HENBUN_REFERENCE names, on the TF-1 shim) produces: re-run the generator into a scratch directory and compare array by
+    array.  Skipped when no reference checkout is named."""
     import subprocess
     import sys
     import pytest
-    if not os.path.isdir("/root/reference/Henbun"):
-        pytest.skip("reference tree not present")
+    ref = os.environ.get("HENBUN_REFERENCE")
+    if not ref or not os.path.isdir(os.path.join(ref, "Henbun")):
+        pytest.skip("no reference checkout: set HENBUN_REFERENCE to a checkout of fujii-team/Henbun")
     env = dict(os.environ, HB_GOLDEN_OUT=str(tmp_path))
     subprocess.run([sys.executable, os.path.join(G, "make_golden.py")], check=True, env=env, stdout=subprocess.DEVNULL,
                    stderr=subprocess.DEVNULL, timeout=600)
