@@ -144,6 +144,13 @@ SIGNATURES = {
     "hb_gp_param_count": (_sz, [C.POINTER(GpConfig)]),
     "hb_gp_elbo_workspace_bytes": (_sz, [C.POINTER(GpConfig)]),
     "hb_gp_elbo_step": (_i, [C.POINTER(GpConfig), _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _sz, _c_f, _c_f]),
+    "hb_gemm_f64": (_i, [_c_f, _ll, _i, _i, _c_f, _ll, _i, _i, _c_f, _ll, _i, _i, _i, _i, C.c_double, C.c_double, _c_f, _sz, _c_f]),
+    "hb_potrf_f64_workspace_bytes": (_sz, [_i]),
+    "hb_potrf_lower_f64": (_i, [_c_f, _ll, _i, _c_f, _sz, _c_f, _c_f]),
+    "hb_potrf_lower_bwd_f64": (_i, [_c_f, _ll, _c_f, _ll, _i, _c_f, _sz, _c_f]),
+    "hb_gp_elbo_f64_workspace_bytes": (_sz, [C.POINTER(GpConfig)]),
+    "hb_gp_elbo_step_f64": (_i, [C.POINTER(GpConfig), _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, C.POINTER(AdamConfig), _c_f,
+                                 _sz, _c_f, _c_f]),
     "hb_comm_unique_id": (_i, [C.c_void_p]),
     "hb_comm_create": (_i, [C.c_void_p, _i, _i, C.POINTER(C.c_void_p)]),
     "hb_comm_destroy": (_i, [C.c_void_p]),
@@ -190,7 +197,8 @@ def load() -> C.CDLL:
 # entry points whose LAST argument is `const hb_options*`, and whole-step entry points whose config struct carries it
 _TRAILING_OPT = ("hb_gemm_ws", "hb_potrf_lower", "hb_potrf_lower_bwd", "hb_trsm_right_lower", "hb_gemm_presplit",
                  "hb_potrf_lower_dist", "hb_potrf_lower_bwd_dist")
-_CFG_OPT = ("hb_gp_elbo_step", "hb_gp_elbo_step_dist", "hb_linop_prepare", "hb_linop_elbo_local", "hb_linop_elbo_update",
+_CFG_OPT = ("hb_gp_elbo_step", "hb_gp_elbo_step_dist", "hb_gp_elbo_step_f64", "hb_gp_elbo_f64_workspace_bytes",
+            "hb_linop_prepare", "hb_linop_elbo_local", "hb_linop_elbo_update",
             "hb_amortised_elbo_step")
 
 

@@ -12,6 +12,7 @@
 // matrices (cond 1e6) put an fp32 factorisation 3 orders of magnitude away from the 1e-5 parity bar.
 #include "kernels.cuh"
 #include "leaf_smem.cuh"
+#include "tmath.cuh"
 
 namespace hb {
 
@@ -22,21 +23,6 @@ constexpr int GS_THREADS = 512;
 template <typename T> struct SmallLimits;
 template <> struct SmallLimits<float> { static constexpr int max_n = 128; };
 template <> struct SmallLimits<double> { static constexpr int max_n = 112; };
-
-template <typename T> __device__ __forceinline__ T t_exp(T x);
-template <> __device__ __forceinline__ float t_exp<float>(float x) { return expf(x); }
-template <> __device__ __forceinline__ double t_exp<double>(double x) { return exp(x); }
-template <typename T> __device__ __forceinline__ T t_log(T x);
-template <> __device__ __forceinline__ float t_log<float>(float x) { return logf(x); }
-template <> __device__ __forceinline__ double t_log<double>(double x) { return log(x); }
-template <typename T> __device__ __forceinline__ T t_sqrt(T x);
-template <> __device__ __forceinline__ float t_sqrt<float>(float x) { return sqrtf(x); }
-template <> __device__ __forceinline__ double t_sqrt<double>(double x) { return sqrt(x); }
-template <typename T> __device__ __forceinline__ T t_softplus(T x) {
-  const T ax = x < T(0) ? -x : x;
-  return (x > T(0) ? x : T(0)) + (T)log1p((double)t_exp<T>(-ax));
-}
-template <typename T> __device__ __forceinline__ T t_sigmoid(T x) { return T(1) / (T(1) + t_exp<T>(-x)); }
 
 template <typename T>
 struct SmallArgs {
@@ -67,7 +53,6 @@ template <typename T>
 __global__ void __launch_bounds__(GS_THREADS, 1) gp_small_step_kernel(const SmallArgs<T> a) {
   extern __shared__ __align__(16) unsigned char gs_smem[];
   const int n = a.n, S = a.S, D = a.D, tid = threadIdx.x;
-  const int tx = tid & 31, ty = tid >> 5;
   const int LD = n | 1;                                  // odd leading dimension: conflict-free column walks
   T* L = reinterpret_cast<T*>(gs_smem);                  // K, then its Cholesky factor (lower)
   T* G = L + (size_t)n * LD;                             // L-bar, then K-bar (lower)
@@ -89,7 +74,6 @@ __global__ void __launch_bounds__(GS_THREADS, 1) gp_small_step_kernel(const Smal
   const T var = t_softplus<T>(*p_var) + T(1e-6);
   const T amp = t_sqrt<T>(kv) * s_q;
   for (int d = tid; d < a.n_ell; d += GS_THREADS) ell[d] = t_softplus<T>(p_ell[d]) + T(1e-6);
-  if (tid == 0) sh_bad = 0;
   __syncthreads();
 
   // ---- K = rbf(X) + jitter I, lower triangle (gp/kernels.py:54-84, 100-101, 110-111) ----
@@ -109,25 +93,8 @@ __global__ void __launch_bounds__(GS_THREADS, 1) gp_small_step_kernel(const Smal
   __syncthreads();
 
   // ---- potrf, right-looking, one column per step (tf.cholesky) ----
-  for (int j = 0; j < n; ++j) {
-    const T d = L[j * LD + j];                           // every thread takes the pivot itself: two barriers per column
-    if (tid == 0 && !(d > T(0)) && sh_bad == 0) sh_bad = j + 1;
-    const T piv = t_sqrt<T>(d > T(0) ? d : T(1)), rp = T(1) / piv;
-    for (int i = j + 1 + tid; i < n; i += GS_THREADS) {
-      const T x = L[i * LD + j] * rp;
-      L[i * LD + j] = x;
-      colv[i] = x;
-    }
-    __syncthreads();
-    if (tid == 0) L[j * LD + j] = piv;
-    // trailing update, 16 x 32 thread grid: rows ty + 16 i, columns tx + 32 k (c <= r)
-    for (int r = j + 1 + ty; r < n; r += 16) {
-      const T lr = colv[r];
-      for (int c = j + 1 + tx; c <= r; c += 32) L[r * LD + c] -= lr * colv[c];
-    }
-    __syncthreads();
-  }
-  if (tid == 0 && sh_bad != 0 && a.err_flag) atomicCAS(a.err_flag, 0, sh_bad);
+  const int bad = potrf_cols_smem<T, GS_THREADS>(L, LD, n, colv, &sh_bad);
+  if (tid == 0 && bad != 0 && a.err_flag) atomicCAS(a.err_flag, 0, bad);
 
   // ---- sampler + one-sample KL (variationals.py:138-146, 183-186, 225-230) ----
   double kl_part = 0.0;
@@ -224,37 +191,7 @@ __global__ void __launch_bounds__(GS_THREADS, 1) gp_small_step_kernel(const Smal
   }
 
   // ---- reverse-mode Cholesky, level-2, in place: G (L-bar) -> dELBO / dK over the stored lower triangle ----
-  for (int j = n - 1; j >= 0; --j) {
-    // reverse of the trailing update of column j: Lbar[r, j] -= sum_c (Abar[r, c] + Abar[c, r]) L[c, j]  (r, c > j):
-    // warp ty owns rows ty + 16 i, its lanes split the columns, one shuffle reduction per row
-    for (int r = j + 1 + ty; r < n; r += 16) {
-      T acc = T(0);
-      for (int c = j + 1 + tx; c < n; c += 32) {
-        const T ab = (c <= r) ? G[r * LD + c] : G[c * LD + r];
-        acc += ab * L[c * LD + j] * ((c == r) ? T(2) : T(1));
-      }
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-      if (tx == 0) colv[r] = acc;
-    }
-    __syncthreads();
-    if (ty == 0) {           // column phase in one warp: scale the column, dot product for the diagonal, no block-wide reduction
-      const T ljj = L[j * LD + j];
-      T dot = T(0);
-      for (int r = j + 1 + tx; r < n; r += 32) {
-        const T lb = G[r * LD + j] - colv[r];            // adjoint of L[r, j]
-        G[r * LD + j] = lb / ljj;                        // reverse of the column scaling: adjoint of A[r, j]
-        dot += lb * L[r * LD + j];
-      }
-#pragma unroll
-      for (int o = 16; o > 0; o >>= 1) dot += __shfl_xor_sync(0xffffffffu, dot, o);
-      if (tx == 0) {
-        const T lbjj = G[j * LD + j] - dot / ljj;        // adjoint of L[j, j]
-        G[j * LD + j] = lbjj / (T(2) * ljj);             // reverse of the square root
-      }
-    }
-    __syncthreads();
-  }
+  potrf_rev_cols_smem<T, GS_THREADS>(L, G, LD, n, colv);
 
   // ---- Gram backward: dELBO / d ell (K recomputed from X; the diagonal does not depend on ell) ----
   {

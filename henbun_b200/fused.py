@@ -243,13 +243,13 @@ class GpElboBinding(object):
 
     SHARED_MIN_N = 4096      # below this a factorisation is a handful of leaves: every rank keeps its own
 
-    # notebook-sized models: the whole step, Adam included, is one persistent CTA (csrc/gp_small.cu)
+    # float_type = float64 (henbunrc:7): the whole step, Adam included, is hb_gp_elbo_step_f64 -- one persistent CTA for
+    # notebook-sized models (csrc/gp_small.cu), the fp64 kernel chain at any larger n (csrc/f64.cu)
     @property
     def fused_adam(self):
-        # in-kernel Adam is the float64 route (henbunrc:7); in fp32 hb_gp_elbo_step already takes the one-CTA kernel for n <= 128 and the
-        # separate Adam launch is faster than Adam inside it (168 vs 180 us)
-        n = self.X.data.shape[0]
-        return self._f64() and n <= int(self.lib.hb_gp_small_max_n(1)) and parallel.world()[0] == 1
+        # in fp32 hb_gp_elbo_step already takes the one-CTA kernel for n <= 128 and the separate Adam launch is faster than Adam
+        # inside it (168 vs 180 us)
+        return self._f64() and parallel.world()[0] == 1
 
     @staticmethod
     def _f64():
@@ -282,11 +282,13 @@ class GpElboBinding(object):
         # potrf_flat / chol_rev_flat) instead of each factoring K itself; samples stay sharded (each rank its own Philox window).
         nranks = parallel.world()[0]
         shared = (not with_adam) and nranks > 1 and n >= self.SHARED_MIN_N and getattr(opt, '_shared_factorisation', True)
-        key = key + (with_adam, f64, shared)
+        key = key + (with_adam, f64, shared, _lib.OPTIONS.small_gp_kernel)     # the option picks the fp64 route and its workspace
         if self._key != key:
             self._env = parallel.block_cyclic_env(shard_samples=True) if shared else None
-            if with_adam:
-                self._wsb = int(self.lib.hb_gp_small_workspace_bytes(C.byref(cfg), 1 if f64 else 0))
+            if f64:
+                self._wsb = int(self.lib.hb_gp_elbo_f64_workspace_bytes(C.byref(cfg)))
+            elif with_adam:
+                self._wsb = int(self.lib.hb_gp_small_workspace_bytes(C.byref(cfg), 0))
             elif shared:
                 self._wsb = int(self.lib.hb_gp_elbo_dist_workspace_bytes(C.byref(cfg), C.byref(self._env)))
             else:
@@ -335,9 +337,9 @@ class GpElboBinding(object):
             cur = opt._flat[:npar]
             self._p64 = torch.where(cur != self._p64.float(), cur.double(), self._p64)
         e = self._eps(eps, count, n, X.device, torch.float64)
-        check(self.lib.hb_gp_small_step_f64(C.byref(cfg), ptr(self._X64), ptr(self._Y64), ptr(self._p64), ptr(e), ptr(self._g64),
-                                            ptr(self._out4), ptr(self._m64), ptr(self._v64), C.byref(adam), ptr(self._ws), self._wsb,
-                                            ptr(err), stream()), "hb_gp_small_step_f64")
+        check(self.lib.hb_gp_elbo_step_f64(C.byref(cfg), ptr(self._X64), ptr(self._Y64), ptr(self._p64), ptr(e), ptr(self._g64),
+                                           ptr(self._out4), ptr(self._m64), ptr(self._v64), C.byref(adam), ptr(self._ws), self._wsb,
+                                           ptr(err), stream()), "hb_gp_elbo_step_f64")
         opt._flat[:npar].copy_(self._p64)
         opt._flat_grad[:npar].copy_(self._g64)
         return self._out4[0]

@@ -322,6 +322,38 @@ size_t hb_gp_elbo_workspace_bytes(const hb_gp_config* cfg);
 int hb_gp_elbo_step(const hb_gp_config* cfg, const float* X, const float* Y, const float* params, const float* eps,
                     float* grads, float* out4, void* ws, size_t ws_bytes, int* err_flag, void* stream);
 
+/* ---- float64 at any size (csrc/f64.cu) --------------------------------------------------------------------------------
+ * The reference's float_type = float64 (henbunrc:7) beyond the one-CTA kernel's n <= 112.  Every pointer is double.
+ *
+ * hb_gemm_f64: C[M,N] = alpha op(A) op(B) + beta C on the fp64 tensor cores (mma.sync f64 -> DMMA).  Layouts and the
+ * triangular masks a_tri / b_tri (0..4) / c_tri (0, 1) as hb_gemm; with c_tri = 1 nothing above the diagonal of C is
+ * written.  beta = 0 does not read C.  ws (optional): outputs of fewer than 74 tiles with K >= 1024 split K over CTAs
+ * into partial tiles of ws (splits * M * N doubles, at most 32 splits) and sum them in a fixed order, so results are
+ * deterministic either way.  No bias, activation or batch.
+ *
+ * hb_potrf_lower_f64 / hb_potrf_lower_bwd_f64: the conventions of hb_potrf_lower / hb_potrf_lower_bwd (lower triangle
+ * only; a non-positive pivot writes 1 + its row into *err_flag; the reverse mode takes G lower = dObj/dL and leaves
+ * dObj/dK in the symmetric-input convention) for one matrix.  The column recursion over 64-column leaves, every
+ * product on hb_gemm_f64, panels solved by substitution (no explicit inverse).  ws of hb_potrf_f64_workspace_bytes(n).
+ *
+ * hb_gp_elbo_step_f64: hb_gp_small_step_f64 at any n, same arguments (adam_m / adam_v NULL: gradient only).  For
+ * n <= hb_gp_small_max_n(1) with opt->small_gp_kernel on (the default) it IS hb_gp_small_step_f64; otherwise, and always
+ * with small_gp_kernel = 0, it runs a chain of kernels: Gram, hb_potrf_lower_f64, sampler + KL, the two S-row
+ * products, log-likelihood, sampler backward, hb_potrf_lower_bwd_f64, Gram backward, scalar chain rules, Adam.  eps NULL
+ * draws the library's Philox stream (the fp32 draw widened to double), the same samples on both routes.
+ * ws of hb_gp_elbo_f64_workspace_bytes(cfg) (which follows cfg->opt to the route). */
+int hb_gemm_f64(const double* A, long long lda, int transA, int a_tri, const double* B, long long ldb, int transB, int b_tri,
+                double* C, long long ldc, int c_tri, int M, int N, int K, double alpha, double beta, void* ws, size_t ws_bytes,
+                void* stream);
+size_t hb_potrf_f64_workspace_bytes(int n);
+int hb_potrf_lower_f64(double* A, long long lda, int n, void* ws, size_t ws_bytes, int* err_flag, void* stream);
+int hb_potrf_lower_bwd_f64(const double* L, long long ldl, double* G, long long ldg, int n, void* ws, size_t ws_bytes,
+                           void* stream);
+size_t hb_gp_elbo_f64_workspace_bytes(const hb_gp_config* cfg);
+int hb_gp_elbo_step_f64(const hb_gp_config* cfg, const double* X, const double* Y, double* params, const double* eps,
+                        double* grads, double* out4, double* adam_m, double* adam_v, const hb_adam_config* adam, void* ws,
+                        size_t ws_bytes, int* err_flag, void* stream);
+
 /* ---- the same step with the factorisation and its reverse mode on a right-looking schedule over column blocks, on one GPU
  * or SHARED BY A GROUP OF GPUs (strong scaling of BASELINE config 3; the reference has no multi-device path, SURVEY.md 8e:
  * tf.cholesky, gp/kernels.py:100-101, and its gradient run on one device).
