@@ -42,6 +42,12 @@ class GpConfig(C.Structure):
                 ("seed", _ull), ("offset", _ull), ("opt", C.POINTER(Options))]
 
 
+class MoeGpConfig(C.Structure):
+    """hb_moe_gp_config: per-expert arrays in the order s, l, r."""
+    _fields_ = [("n", _i), ("D", _i), ("S", _i), ("n_ell", _i * 3), ("q_fullrank", _i * 3), ("jitter", C.c_double),
+                ("seed", _ull), ("offset", _ull * 3), ("opt", C.POINTER(Options))]
+
+
 class Dist(C.Structure):
     """hb_dist: this rank's place in a column-block-cyclic factorisation (comm from hb_comm_create; NULL when world == 1)."""
     _fields_ = [("comm", C.c_void_p), ("rank", _i), ("world", _i), ("block", _i), ("shard_samples", _i), ("batch", _i), ("block_bwd", _i), ("turn", _i)]
@@ -151,6 +157,10 @@ SIGNATURES = {
     "hb_gp_elbo_f64_workspace_bytes": (_sz, [C.POINTER(GpConfig)]),
     "hb_gp_elbo_step_f64": (_i, [C.POINTER(GpConfig), _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, C.POINTER(AdamConfig), _c_f,
                                  _sz, _c_f, _c_f]),
+    "hb_moe_gp_param_count": (_sz, [C.POINTER(MoeGpConfig)]),
+    "hb_moe_gp_f64_workspace_bytes": (_sz, [C.POINTER(MoeGpConfig)]),
+    "hb_moe_gp_elbo_step_f64": (_i, [C.POINTER(MoeGpConfig), _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _c_f,
+                                     C.POINTER(AdamConfig), _c_f, _sz, _c_f, _c_f]),
     "hb_comm_unique_id": (_i, [C.c_void_p]),
     "hb_comm_create": (_i, [C.c_void_p, _i, _i, C.POINTER(C.c_void_p)]),
     "hb_comm_destroy": (_i, [C.c_void_p]),
@@ -198,6 +208,7 @@ def load() -> C.CDLL:
 _TRAILING_OPT = ("hb_gemm_ws", "hb_potrf_lower", "hb_potrf_lower_bwd", "hb_trsm_right_lower", "hb_gemm_presplit",
                  "hb_potrf_lower_dist", "hb_potrf_lower_bwd_dist")
 _CFG_OPT = ("hb_gp_elbo_step", "hb_gp_elbo_step_dist", "hb_gp_elbo_step_f64", "hb_gp_elbo_f64_workspace_bytes",
+            "hb_moe_gp_elbo_step_f64", "hb_moe_gp_f64_workspace_bytes",
             "hb_linop_prepare", "hb_linop_elbo_local", "hb_linop_elbo_update",
             "hb_amortised_elbo_step")
 

@@ -12,6 +12,7 @@
 //               ill-conditioned Gram matrices fp64 is chosen for.
 #include "../../include/henbun_b200.h"
 #include "gemm.cuh"
+#include "f64.cuh"
 #include "kernels.cuh"
 #include "tmath.cuh"
 #include <algorithm>
@@ -21,7 +22,6 @@ namespace hb {
 namespace {
 
 inline cudaStream_t S_(void* s) { return reinterpret_cast<cudaStream_t>(s); }
-inline size_t align256(size_t x) { return (x + 255) / 256 * 256; }
 
 // ------------------------------------------------------------------------------------------------------------------
 // fp64 GEMM:  C[M,N] = alpha op(A) op(B) + beta C,  masks as GemmParams (gemm.cuh)
@@ -374,6 +374,8 @@ __global__ void __launch_bounds__(PS64_ROWS) panel_solve_f64_kernel(const double
   }
 }
 
+}  // namespace
+
 int ensure_attrs64() {
   static bool done = false;
   if (done) return HB_OK;
@@ -389,16 +391,11 @@ int ensure_attrs64() {
 // ------------------------------------------------------------------------------------------------------------------
 // the column recursion (linalg.cu: potrf_cols / chol_rev_cols) with every product on the fp64 GEMM
 // ------------------------------------------------------------------------------------------------------------------
-struct Ctx64 {
-  cudaStream_t st;
-  int* err;
-  void* ws;                // split-K partial tiles
-  size_t ws_bytes;
-};
-
-constexpr size_t kSplitWsBytes = (size_t)8 << 20;       // 32 partial 128 x 128 tiles, 64 partial 64 x 64 ones
+namespace {
 
 inline int split64(int w) { return ((cdiv(w, NB64) + 1) / 2) * NB64; }
+
+}  // namespace
 
 int gemm64(const Ctx64& c, const double* A, long long lda, int transA, int a_tri, const double* B, long long ldb, int transB,
            int b_tri, double* C, long long ldc, int c_tri, int M, int N, int K, double alpha, double beta) {
@@ -406,12 +403,16 @@ int gemm64(const Ctx64& c, const double* A, long long lda, int transA, int a_tri
   return gemm_f64(p, c.ws, c.ws_bytes, c.st);
 }
 
+namespace {
+
 int panel_solve64(const Ctx64& c, const double* D, long long ldd, double* Bp, long long ldb, int m, int w, bool trans, double alpha) {
   if (trans) panel_solve_f64_kernel<true><<<cdiv(m, PS64_ROWS), PS64_ROWS, kPanel64Smem, c.st>>>(D, ldd, Bp, ldb, m, w, alpha);
   else panel_solve_f64_kernel<false><<<cdiv(m, PS64_ROWS), PS64_ROWS, kPanel64Smem, c.st>>>(D, ldd, Bp, ldb, m, w, alpha);
   HB_CHECK_LAUNCH();
   return HB_OK;
 }
+
+}  // namespace
 
 int potrf_cols64(const Ctx64& c, double* A, long long lda, int c0, int w, int n) {
   double* D = A + (long long)c0 * lda + c0;
@@ -465,6 +466,8 @@ int chol_rev_cols64(const Ctx64& c, const double* L, long long ldl, double* G, l
   return chol_rev_cols64(c, L, ldl, G, ldg, c0, w1, n);
 }
 
+namespace {
+
 size_t potrf64_ws_bytes(int n) { return n > NB64 ? kSplitWsBytes + 256 : 0; }
 
 int make_ctx64(Ctx64& c, int n, void* ws, size_t ws_bytes, int* err, cudaStream_t st) {
@@ -495,10 +498,6 @@ int potrf_lower_bwd_f64(const double* L, long long ldl, double* G, long long ldg
 // the rest of the GP step in double (the formulas of gp_small.cu's step, as separate kernels)
 // sc: [0] scale s, [1] k_var, [2] var, [3] amp = sqrt(k_var) s, [4] loglik, [5] sum E^2, [6] sum E Fraw, [7] kl, [8..) ell
 // ------------------------------------------------------------------------------------------------------------------
-constexpr int SC_ELL = 8;
-constexpr int kGramBwdBlocks = 296;
-constexpr int RED_THREADS = 1024;
-
 __global__ void gp64_prep_kernel(const double* p_scale, const double* p_ell, int n_ell, const double* p_kvar, const double* p_var,
                                  double* sc) {
   if (threadIdx.x == 0) {
@@ -507,6 +506,8 @@ __global__ void gp64_prep_kernel(const double* p_scale, const double* p_ell, int
   }
   for (int d = threadIdx.x; d < n_ell; d += blockDim.x) sc[SC_ELL + d] = t_softplus<double>(p_ell[d]) + 1e-6;
 }
+
+}  // namespace
 
 // K = rbf(X) + jitter I, 32 x 32 tiles on and below the diagonal
 __global__ void gp64_gram_kernel(const double* X, int n, int D, const double* sc, int n_ell, double jitter, double* K) {
@@ -553,6 +554,8 @@ __global__ void __launch_bounds__(RED_THREADS) gp64_kl_kernel(const double* p_sq
   if (threadIdx.x == 0) sc[7] = -0.5 * v[0];
 }
 
+namespace {
+
 // log-likelihood of Y under F = amp Fraw, sum E^2, sum E Fraw, residual R = E / var / S: one CTA, fixed order
 __global__ void __launch_bounds__(RED_THREADS) gp64_loglik_kernel(const double* Fraw, const double* Y, int n, int S, double* R,
                                                                 double* sc) {
@@ -569,6 +572,8 @@ __global__ void __launch_bounds__(RED_THREADS) gp64_loglik_kernel(const double* 
   block_sum<3>(v, red);
   if (threadIdx.x == 0) { sc[4] = v[0]; sc[5] = v[1]; sc[6] = v[2]; }
 }
+
+}  // namespace
 
 // z-bar = amp W - Z / S  (W = R L)
 __global__ void gp64_zbar_kernel(const double* W, const double* Z, const double* sc, long long total, int S, double* Zb) {
@@ -629,6 +634,8 @@ __global__ void __launch_bounds__(256) gp64_gram_bwd_kernel(const double* G, con
   }
 }
 
+namespace {
+
 // lengthscale gradient (K-bar came without the factor amp: the reverse-mode Cholesky is linear in L-bar), scalar chain rules,
 // the ELBO
 __global__ void gp64_scalar_bwd_kernel(const double* sc, const double* red, int nblk, int n_ell, int n, int S, const double* p_scale,
@@ -652,6 +659,8 @@ __global__ void gp64_scalar_bwd_kernel(const double* sc, const double* red, int 
   }
 }
 
+}  // namespace
+
 // TF-1 Adam on -ELBO (model.py:206,220); the strict upper triangle of a full-rank q_sqrt never moves
 __global__ void gp64_adam_kernel(double* params, const double* grads, double* m, double* v, long long npar, int n, int full,
                                  const int* step_dev, int step_host, double lr, double b1, double b2, double eps, double grad_scale) {
@@ -670,6 +679,8 @@ __global__ void gp64_adam_kernel(double* params, const double* grads, double* m,
     params[i] -= lr_t * mm / (sqrt(vv) + eps);
   }
 }
+
+namespace {
 
 struct Gp64Layout {
   size_t off_K, off_G, off_Z, off_F, off_R, off_W, off_U, off_sc, off_red, off_potrf, total;

@@ -166,7 +166,40 @@ def _split_elbo(tree, model):
     return yv, f, vv, kl.args[1]
 
 
-class GpElboBinding(object):
+class _Float64Masters(object):
+    """float_type = float64 (henbunrc:7) for a whole-step entry point whose parameters are packed at the start of the
+    Optimizer's flat buffers: fp64 master copies of the parameters, their gradient and the Adam moments live in the binding,
+    and the fp32 flat buffer mirrors them after every step (so .value, save() and the eager evaluation keep working)."""
+    _p64 = None
+    _src64 = None
+
+    def _data64(self, dev):
+        """fp64 device copies of X and Y, refreshed when new data is fed."""
+        if self._src64 is None or self._src64[0] is not self.X.data or self._src64[1] is not self.Y.data:
+            self._X64 = torch.as_tensor(np.ascontiguousarray(self.X.data, dtype=np.float64)).to(dev)
+            self._Y64 = torch.as_tensor(np.ascontiguousarray(self.Y.data, dtype=np.float64)).to(dev).reshape(-1)
+            self._src64 = (self.X.data, self.Y.data)
+        return self._X64, self._Y64
+
+    def _pull64(self, opt, npar, dev):
+        """Masters before a step: created from the fp32 buffers at the first step, afterwards taking every entry of the
+        fp32 mirror that was edited from outside since the last step."""
+        if self._p64 is None:
+            self._p64 = opt._flat[:npar].double()
+            self._g64 = torch.zeros(npar, dtype=torch.float64, device=dev)
+            self._m64 = opt._m[:npar].double(); self._v64 = opt._v[:npar].double()
+        else:
+            # entries of the fp32 mirror that no longer equal the rounded master were edited from outside since the last
+            # step (an assignment, restore(), another Optimizer over the same variables): the master takes them
+            cur = opt._flat[:npar]
+            self._p64 = torch.where(cur != self._p64.float(), cur.double(), self._p64)
+
+    def _push64(self, opt, npar):
+        opt._flat[:npar].copy_(self._p64)
+        opt._flat_grad[:npar].copy_(self._g64)
+
+
+class GpElboBinding(_Float64Masters):
     """notebooks/GaussianProcess.ipynb:109-148 recognised in a traced objective:
         y_fit = matmul(kern.Cholesky(X), q) * sqrt(k_var);  ELBO = reduce_sum(gaussian(Y, y_fit, var)) - KL()
     with q = variationals.Gaussian([n, 1]) (diagonal or fullrank), kern = UnitRBF.  One call of hb_gp_elbo_step writes the
@@ -320,28 +353,198 @@ class GpElboBinding(object):
                                             ptr(opt._m), ptr(opt._v), C.byref(adam), ptr(self._ws), self._wsb, ptr(err), stream()),
                   "hb_gp_small_step")
             return self._out4[0]
-        # float_type = float64 (henbunrc:7): fp64 master copies of parameters / moments live here, the Optimizer's fp32 flat
-        # buffer mirrors them after every step (so .value, save() and the eager evaluation keep working)
+        # float_type = float64 (henbunrc:7): fp64 master copies of parameters / moments (_Float64Masters)
         dev = X.device
-        if self._src64 is None or self._src64[0] is not self.X.data or self._src64[1] is not self.Y.data:
-            self._X64 = torch.as_tensor(np.ascontiguousarray(self.X.data, dtype=np.float64)).to(dev)
-            self._Y64 = torch.as_tensor(np.ascontiguousarray(self.Y.data, dtype=np.float64)).to(dev).reshape(-1)
-            self._src64 = (self.X.data, self.Y.data)
-        if self._p64 is None:
-            self._p64 = opt._flat[:npar].double()
-            self._g64 = torch.zeros(npar, dtype=torch.float64, device=dev)
-            self._m64 = opt._m[:npar].double(); self._v64 = opt._v[:npar].double()
-        else:
-            # entries of the fp32 mirror that no longer equal the rounded master were edited from outside since the last
-            # step (an assignment, restore(), another Optimizer over the same variables): the master takes them
-            cur = opt._flat[:npar]
-            self._p64 = torch.where(cur != self._p64.float(), cur.double(), self._p64)
+        X64, Y64 = self._data64(dev)
+        self._pull64(opt, npar, dev)
         e = self._eps(eps, count, n, X.device, torch.float64)
-        check(self.lib.hb_gp_elbo_step_f64(C.byref(cfg), ptr(self._X64), ptr(self._Y64), ptr(self._p64), ptr(e), ptr(self._g64),
+        check(self.lib.hb_gp_elbo_step_f64(C.byref(cfg), ptr(X64), ptr(Y64), ptr(self._p64), ptr(e), ptr(self._g64),
                                            ptr(self._out4), ptr(self._m64), ptr(self._v64), C.byref(adam), ptr(self._ws), self._wsb,
                                            ptr(err), stream()), "hb_gp_elbo_step_f64")
-        opt._flat[:npar].copy_(self._p64)
-        opt._flat_grad[:npar].copy_(self._g64)
+        self._push64(opt, npar)
+        return self._out4[0]
+
+
+def _operands(node, op):
+    """(a, b) of a binary `op` node, or None."""
+    from .trace import Sym
+    if isinstance(node, Sym) and node.op == op and len(node.args) == 2:
+        return node.args
+    return None
+
+
+def _commuted(node, op, first):
+    """Operands of a commutative `op` node as (x, y) with first(x) true, trying both orders; None if neither fits."""
+    ab = _operands(node, op)
+    if ab is None:
+        return None
+    for x, y in (ab, ab[::-1]):
+        if first(x):
+            return x, y
+    return None
+
+
+def _gp_projection(node):
+    """matmul(kern.Cholesky(X), q) with a UnitRBF kernel (Log1pe lengthscales) and a variationals.Gaussian q of shape [n, 1]
+    -> (kern, X data variable, q), else None."""
+    from .trace import Sym
+    from .variationals import Gaussian
+    from .gp.kernels import UnitRBF
+    from .param import Variable
+    from . import transforms
+    if not (isinstance(node, Sym) and node.op == 'matmul' and not node.kw['ta'] and not node.kw['tb']):
+        return None
+    ch, smp = node.args
+    if not (isinstance(ch, Sym) and ch.op == 'cholesky' and isinstance(smp, Sym) and smp.op == 'sample'):
+        return None
+    kern, Xs = ch.args
+    X, q = _leaf(Xs, 'data'), smp.args[0]
+    if X is None or type(kern) is not UnitRBF or type(q) is not Gaussian or smp.args[1] is not None:
+        return None
+    ell = object.__getattribute__(kern, 'lengthscales')
+    if not (isinstance(ell, Variable) and ell.is_parameter and isinstance(ell.transform, transforms.Log1pe)
+            and abs(float(ell.transform._lower) - 1e-6) < 1e-12):
+        return None
+    if q.n_layers or q.n_batch is not None or q.is_local or not isinstance(q.transform, transforms.Identity):
+        return None
+    if not _is_positive_scalar(object.__getattribute__(q, 'scale')):
+        return None
+    return kern, X, q
+
+
+class MixtureGpElboBinding(_Float64Masters):
+    """notebooks/Expert_GPR.ipynb:101-149 (BASELINE config 2) recognised in a traced objective under float_type = float64:
+        f_s = matmul(kern_s.Cholesky(X), q_s);  f_l = matmul(kern_l.Cholesky(X), q_l)
+        f_r = matmul(kern_r.Cholesky(X), q_r) * sqrt(k_var_r);  fraction = sigmoid(f_r)
+        ELBO = reduce_sum(gaussian(Y, (fraction * f_s + (1 - fraction) * f_l) * k_var, var)) - KL()
+    (either operand order of every mul and add) with three distinct UnitRBF kernels and three distinct
+    variationals.Gaussian([n, 1]).  One call of hb_moe_gp_elbo_step_f64 (csrc/moe64.cu) runs the step, TF-1 Adam included,
+    on fp64 master copies (_Float64Masters) packed as [q_s.q_mu | q_s.q_sqrt | q_s.scale | kern_s.lengthscales | the same for
+    l and r | k_var | k_var_r | var].  `qs` lists the variationals in the order the objective samples them, the order of
+    their Philox windows on the eager tape."""
+
+    fused_adam = True
+
+    def __init__(self, model, experts, k_var, k_var_r, var, X, Y, qs):
+        self.model, self.experts, self.X, self.Y, self.qs = model, experts, X, Y, qs
+        self.k_var, self.k_var_r, self.var = k_var, k_var_r, var
+        g = object.__getattribute__
+        order = []
+        for kern, q in experts:
+            order += [g(q, 'q_mu'), g(q, 'q_sqrt'), g(q, 'scale'), g(kern, 'lengthscales')]
+        self.var_order = order + [k_var, k_var_r, var]
+        self.lib = _lib.load()
+        self._key = None
+
+    @staticmethod
+    def match(tree, model):
+        from .trace import Sym, draws
+        from .param import MinibatchData, graph_key
+        from ._settings import settings
+        if str(settings.dtypes.float_type) != 'float64' or parallel.world()[0] != 1:
+            return None
+        parts = _split_elbo(tree, model)
+        if parts is None:
+            return None
+        Y, f, var, kl_coll = parts
+        if kl_coll not in (None, graph_key.VARIABLES):
+            return None
+        param = lambda x: _leaf(x, 'param') is not None and _is_positive_scalar(_leaf(x, 'param'))
+        sig = lambda x: isinstance(x, Sym) and x.op == 'sigmoid'
+        one_minus = lambda x: (isinstance(x, Sym) and x.op == 'sub' and isinstance(x.args[0], (int, float))
+                               and x.args[0] == 1 and sig(x.args[1]))
+        # (mixture) * k_var
+        mk = _commuted(f, 'mul', lambda x: not param(x))
+        if mk is None or not param(mk[1]):
+            return None
+        mix, k_var = mk[0], _leaf(mk[1], 'param')
+        # sigmoid(f_r) * f_s + (1 - sigmoid(f_r)) * f_l
+        sl = _commuted(mix, 'add', lambda x: _commuted(x, 'mul', sig) is not None)
+        if sl is None:
+            return None
+        gate_s, f_s = _commuted(sl[0], 'mul', sig)
+        gl = _commuted(sl[1], 'mul', one_minus)
+        if gl is None:
+            return None
+        gate_l, f_l = gl[0].args[1], gl[1]
+        # f_r = matmul(kern_r.Cholesky(X), q_r) * sqrt(k_var_r), the same gate on both experts
+        gates = []
+        for gate in (gate_s, gate_l):
+            fr = _commuted(gate.args[0], 'mul', lambda x: isinstance(x, Sym) and x.op == 'sqrt' and param(x.args[0]))
+            if fr is None:
+                return None
+            gates.append((_leaf(fr[0].args[0], 'param'), _gp_projection(fr[1])))
+        if gates[0][1] is None or gates[1][1] is None or gates[0][0] is not gates[1][0] or \
+                any(a is not b for a, b in zip(gates[0][1], gates[1][1])):
+            return None
+        k_var_r, proj_r = gates[0]
+        projs = [_gp_projection(f_s), _gp_projection(f_l), proj_r]
+        if any(pr is None for pr in projs):
+            return None
+        kerns, Xs, qs = zip(*projs)
+        X = Xs[0]
+        if any(x is not X for x in Xs) or isinstance(X, MinibatchData) or isinstance(Y, MinibatchData):
+            return None
+        if len({id(k) for k in kerns}) != 3 or len({id(q) for q in qs}) != 3:
+            return None
+        if len({id(v) for v in (k_var, k_var_r, var)}) != 3:
+            return None
+        if X.data.ndim != 2 or Y.data.shape != (X.data.shape[0], 1):
+            return None
+        n, D = X.data.shape
+        if D > 32 or any(list(q._shape) != [n, 1] for q in qs):
+            return None
+        if any(int(np.prod(object.__getattribute__(k, 'lengthscales')._host.shape)) not in (1, D) for k in kerns):
+            return None
+        found = _variationals_of(model)          # KL() must be exactly these three variationals'
+        if len(found) != 3 or {id(q) for q in found} != {id(q) for q in qs}:
+            return None
+        order = [q for q in draws() if any(q is r for r in qs)]
+        if len(order) != 3:
+            return None
+        return MixtureGpElboBinding(model, list(zip(kerns, qs)), k_var, k_var_r, var, X, Y, order)
+
+    def per_sample(self):
+        return int(self.X.data.shape[0])
+
+    def step(self, opt, count, eps, seed, offsets, world=None):
+        """One ELBO + gradient + Adam step.  eps / offsets: one per variational of `qs` (an injected [count, n] draw or None;
+        the Philox stream position of a variational without one)."""
+        from . import ops
+        X = self.X.tensor()
+        n, D = X.shape
+        dev = X.device
+        role = {id(q): i for i, (_, q) in enumerate(self.experts)}       # s, l, r
+        e64, off = [None] * 3, [0] * 3
+        for q, e, o in zip(self.qs, eps, offsets):
+            i = role[id(q)]
+            e64[i] = None if e is None else (torch.as_tensor(np.asarray(e), dtype=torch.float64) if not isinstance(e, torch.Tensor)
+                                             else e).to(dev, torch.float64).reshape(count, n).contiguous()
+            off[i] = int(o)
+        n_ell = [int(np.prod(object.__getattribute__(k, 'lengthscales')._host.shape)) for k, _ in self.experts]
+        full = [1 if q.q_shape == 'fullrank' else 0 for _, q in self.experts]
+        cfg = _lib.MoeGpConfig(int(n), int(D), int(count), (C.c_int * 3)(*n_ell), (C.c_int * 3)(*full),
+                               float(opt._compiled_settings.numerics.jitter_level), int(seed), (C.c_ulonglong * 3)(*off))
+        key = (int(n), int(D), int(count), tuple(n_ell), tuple(full))
+        if self._key != key:
+            self._wsb = int(self.lib.hb_moe_gp_f64_workspace_bytes(C.byref(cfg)))
+            self._ws = torch.empty(self._wsb, dtype=torch.uint8, device=dev)
+            self._out4 = torch.zeros(4, dtype=torch.float64, device=dev)
+            self._p64 = None
+            self._key = key
+        npar = int(self.lib.hb_moe_gp_param_count(C.byref(cfg)))
+        X64, Y64 = self._data64(dev)
+        self._pull64(opt, npar, dev)
+        err = ops.err_flag(dev)
+        check(self.lib.hb_increment_i32(ptr(opt._step), stream()), "hb_increment_i32")
+        o = opt.optimizer
+        adam = _lib.AdamConfig(float(o.learning_rate), float(o.beta1), float(o.beta2), float(o.epsilon), -1.0,
+                               C.c_void_p(opt._step.data_ptr()), 0)
+        check(self.lib.hb_moe_gp_elbo_step_f64(C.byref(cfg), ptr(X64), ptr(Y64), ptr(self._p64), ptr(e64[0]), ptr(e64[1]),
+                                               ptr(e64[2]), ptr(self._g64), ptr(self._out4), ptr(self._m64), ptr(self._v64),
+                                               C.byref(adam), ptr(self._ws), self._wsb, ptr(err), stream()),
+              "hb_moe_gp_elbo_step_f64")
+        self._push64(opt, npar)
         return self._out4[0]
 
 
@@ -558,7 +761,7 @@ def _split_elbo_mb(tree, model):
     return yv, f, vv, kl.args[1]
 
 
-BINDINGS = (GpElboBinding, LinopElboBinding, AmortisedElboBinding)
+BINDINGS = (GpElboBinding, MixtureGpElboBinding, LinopElboBinding, AmortisedElboBinding)
 
 
 def bind(tree, model):

@@ -374,6 +374,12 @@ class Optimizer(object):
         with settings.temp_settings(self._compiled_settings):
             m._begin_run(count, eps, shard=(first, total))
         ctx = m._run_ctx
+        qs = getattr(b, 'qs', None)
+        if qs is not None:
+            # several variationals: one eps (or Philox window, taken in the order the tape takes them) per variational
+            es = [None if not eps else eps.get(q, None) for q in qs]
+            offsets = [ctx.take_sharded(b.per_sample()) if e is None else 0 for e in es]
+            return b.step(self, count, es, ctx.seed, offsets, world)
         q = b.q
         e = None if not eps else eps.get(q, None)
         offset = ctx.take_sharded(b.per_sample()) if e is None else 0

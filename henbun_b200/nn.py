@@ -15,6 +15,9 @@ from ._settings import settings
 
 def sigmoid(x, name=None):
     import torch
+    from . import trace as _trace
+    if isinstance(x, _trace.Sym):
+        return _trace.Sym('sigmoid', x)
     return torch.sigmoid(x)
 
 

@@ -2,24 +2,33 @@
 (Henbun/model.py:217-221: ``method_op = likelihood_method(model)`` inside tf_mode builds ONE TensorFlow graph that
 every ``session.run`` replays).  ``Optimizer.compile`` runs the objective once with every parameter / data / sample
 replaced by a ``Sym`` leaf; the ops of the hot path (tf.matmul, kern.Cholesky, densities.gaussian, tf.reduce_sum,
-tf.sqrt, NeuralNet calls, LOCAL feeds, KL()) build an expression tree instead of launching kernels.  ``fused.py``
-matches that tree against the graphs that have a whole-step C entry point (variational GP regression, the linear
-operator model, the amortised encoder/decoder model).  Anything the tracer does not understand raises, and the
-Optimizer keeps the eager tape path -- tracing never changes results, it only selects the faster executor."""
+tf.sqrt, tf.sigmoid, NeuralNet calls, LOCAL feeds, KL()) build an expression tree instead of launching kernels.
+``fused.py`` matches that tree against the graphs that have a whole-step C entry point (variational GP regression, the
+mixture of GP experts in float64, the linear operator model, the amortised encoder/decoder model).  Anything the tracer
+does not understand raises, and the Optimizer keeps the eager tape path -- tracing never changes results, it only selects
+the faster executor."""
 from __future__ import annotations
 
 import contextlib
 
 _ACTIVE = [False]
+_DRAWS = []          # variationals of the current (or last) trace, in the order their first 'sample' node was created
 
 
 def active() -> bool:
     return _ACTIVE[0]
 
 
+def draws():
+    """Variationals sampled by the last traced objective, in the order it first sampled them.  The eager tape takes each
+    variational's Philox window at its first sample, so this is the order of those windows."""
+    return list(_DRAWS)
+
+
 @contextlib.contextmanager
 def tracing():
     _ACTIVE[0] = True
+    del _DRAWS[:]
     try:
         yield
     finally:
@@ -37,6 +46,8 @@ class Sym(object):
 
     def __init__(self, op, *args, **kw):
         self.op, self.args, self.kw = op, args, kw
+        if op == 'sample' and _ACTIVE[0] and not any(q is args[0] for q in _DRAWS):
+            _DRAWS.append(args[0])
 
     def _bin(self, op, other, swap=False):
         if not isinstance(other, (Sym, int, float)):

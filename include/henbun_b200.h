@@ -354,6 +354,33 @@ int hb_gp_elbo_step_f64(const hb_gp_config* cfg, const double* X, const double* 
                         double* grads, double* out4, double* adam_m, double* adam_v, const hb_adam_config* adam, void* ws,
                         size_t ws_bytes, int* err_flag, void* stream);
 
+/* ---- float64 mixture-of-experts GP regression (csrc/moe64.cu) ----------------------------------------------------------
+ * notebooks/Expert_GPR.ipynb:101-149 (BASELINE config 2), S-sample mean, every pointer double: experts s, l and gate r,
+ *   f_e = matmul(kern_e.Cholesky(X), q_e),  frac = sigmoid(f_r * sqrt(k_var_r)),
+ *   ELBO = sum gaussian(Y, (frac f_s + (1 - frac) f_l) * k_var, var) - KL()
+ * with q_e = variationals.Gaussian(shape=[n,1], q_fullrank[e]) and kern_e = UnitRBF (n_ell[e] = 1 or D lengthscales).
+ * params / grads packing (free space): [ q_mu | q_sqrt | scale | lengthscales ] for s, then l, then r (each segment laid
+ * out as hb_gp_config's packing up to its lengthscales), then [ k_var | k_var_r | var ].  out4 = { ELBO, loglik_sum, kl_sum over the three, 0 }.
+ * eps_e: [S,n] or NULL (the library's Philox stream at (seed, offset[e]), the fp32 draw widened to double; offset[e] a
+ * multiple of 4).  adam_m / adam_v NULL: gradient only; otherwise the TF-1 Adam update of hb_gp_elbo_step_f64 follows.
+ * A non-positive pivot in any expert's factorisation writes 1 + its row into *err_flag; the three factorisations run
+ * concurrently, so when several fail the row is that of whichever got there first, and the expert is not identified.  The three GP chains run
+ * concurrently on two side streams forked from `stream` and joined back into it; results are bitwise repeatable and
+ * `stream` has waited on all of the work when the call returns.  D <= 32.  ws of hb_moe_gp_f64_workspace_bytes(cfg). */
+typedef struct {
+  int n, D, S;
+  int n_ell[3];                        /* 1 or D; experts s, l, gate r */
+  int q_fullrank[3];
+  double jitter;
+  unsigned long long seed, offset[3];  /* Philox window per variational; each a multiple of 4 when its eps is NULL */
+  const hb_options* opt;               /* NULL = defaults */
+} hb_moe_gp_config;
+size_t hb_moe_gp_param_count(const hb_moe_gp_config* cfg);
+size_t hb_moe_gp_f64_workspace_bytes(const hb_moe_gp_config* cfg);
+int hb_moe_gp_elbo_step_f64(const hb_moe_gp_config* cfg, const double* X, const double* Y, double* params, const double* eps_s,
+                            const double* eps_l, const double* eps_r, double* grads, double* out4, double* adam_m,
+                            double* adam_v, const hb_adam_config* adam, void* ws, size_t ws_bytes, int* err_flag, void* stream);
+
 /* ---- the same step with the factorisation and its reverse mode on a right-looking schedule over column blocks, on one GPU
  * or SHARED BY A GROUP OF GPUs (strong scaling of BASELINE config 3; the reference has no multi-device path, SURVEY.md 8e:
  * tf.cholesky, gp/kernels.py:100-101, and its gradient run on one device).
