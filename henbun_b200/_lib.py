@@ -138,6 +138,10 @@ SIGNATURES = {
     "hb_linop_elbo_local": (_i, [C.POINTER(LinopConfig), _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _sz, _c_f]),
     "hb_linop_elbo_update": (_i, [C.POINTER(LinopConfig), _c_f, _c_f, _c_f, _c_f, _c_f, _fl, _fl, _fl, _fl, _c_f, _i,
                                   _c_f, _c_f, _sz, _c_f]),
+    "hb_linop_f64_workspace_bytes": (_sz, [C.POINTER(LinopConfig)]),
+    "hb_linop_elbo_local_f64": (_i, [C.POINTER(LinopConfig), _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _sz, _c_f]),
+    "hb_linop_elbo_update_f64": (_i, [C.POINTER(LinopConfig), _c_f, _c_f, _c_f, _c_f, _c_f, C.POINTER(AdamConfig), _c_f, _c_f,
+                                      _sz, _c_f]),
     "hb_amortised_param_count": (_sz, [C.POINTER(AmortisedConfig)]),
     "hb_amortised_workspace_bytes": (_sz, [C.POINTER(AmortisedConfig)]),
     "hb_amortised_elbo_step": (_i, [C.POINTER(AmortisedConfig), _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _sz, _c_f]),

@@ -169,9 +169,11 @@ def _split_elbo(tree, model):
 class _Float64Masters(object):
     """float_type = float64 (henbunrc:7) for a whole-step entry point whose parameters are packed at the start of the
     Optimizer's flat buffers: fp64 master copies of the parameters, their gradient and the Adam moments live in the binding,
-    and the fp32 flat buffer mirrors them after every step (so .value, save() and the eager evaluation keep working)."""
+    and the fp32 flat buffer mirrors them after every step (so .value, save() and the eager evaluation keep working).
+    A binding whose entry point never writes a flat gradient sets _grad64 = False: no fp64 gradient is allocated or pushed."""
     _p64 = None
     _src64 = None
+    _grad64 = True
 
     def _data64(self, dev):
         """fp64 device copies of X and Y, refreshed when new data is fed."""
@@ -186,7 +188,7 @@ class _Float64Masters(object):
         fp32 mirror that was edited from outside since the last step."""
         if self._p64 is None:
             self._p64 = opt._flat[:npar].double()
-            self._g64 = torch.zeros(npar, dtype=torch.float64, device=dev)
+            self._g64 = torch.zeros(npar, dtype=torch.float64, device=dev) if self._grad64 else None
             self._m64 = opt._m[:npar].double(); self._v64 = opt._v[:npar].double()
         else:
             # entries of the fp32 mirror that no longer equal the rounded master were edited from outside since the last
@@ -196,7 +198,8 @@ class _Float64Masters(object):
 
     def _push64(self, opt, npar):
         opt._flat[:npar].copy_(self._p64)
-        opt._flat_grad[:npar].copy_(self._g64)
+        if self._grad64:
+            opt._flat_grad[:npar].copy_(self._g64)
 
 
 class GpElboBinding(_Float64Masters):
@@ -548,18 +551,25 @@ class MixtureGpElboBinding(_Float64Masters):
         return self._out4[0]
 
 
-class LinopElboBinding(object):
+class LinopElboBinding(_Float64Masters):
     """BASELINE config 5 recognised in a traced objective:
         f = matmul(q, A, transpose_b=True);  ELBO = reduce_sum(gaussian(y, f, var)) - KL()
     with q = variationals.Normal([n], 'fullrank').  The step runs hb_linop_elbo_local / _update on the Optimizer's flat
-    buffers (packing [q_sqrt | q_mu | var]); the q_sqrt gradient is formed and consumed by Adam in one pass."""
+    buffers (packing [q_sqrt | q_mu | var]); the q_sqrt gradient is formed and consumed by Adam in one pass.
+    Under float_type = float64 (henbunrc:7) with one process (`f64`, fixed when compile() binds), the step is the fp64 pair
+    hb_linop_elbo_local_f64 / _update_f64 (csrc/linop64.cu) on fp64 master copies (_Float64Masters) and fp64 device copies
+    of A and y."""
 
-    def __init__(self, model, q, var, A, y):
+    _grad64 = False                     # neither route writes the flat gradient: no n x n fp64 gradient either
+
+    def __init__(self, model, q, var, A, y, f64=False):
         self.model, self.q, self.var, self.A, self.y = model, q, var, A, y
         g = object.__getattribute__
         self.var_order = [g(q, 'q_sqrt'), g(q, 'q_mu'), var]
         self.fused_adam = True
+        self.f64 = bool(f64)
         self._st = None
+        self._key64 = None
 
     @staticmethod
     def match(tree, model):
@@ -589,12 +599,58 @@ class LinopElboBinding(object):
             return None
         if _variationals_of(model) != [q]:
             return None
-        return LinopElboBinding(model, q, var, A, y)
+        from ._settings import settings
+        f64 = str(settings.dtypes.float_type) == 'float64' and parallel.world()[0] == 1
+        return LinopElboBinding(model, q, var, A, y, f64=f64)
 
     def per_sample(self):
         return int(self.A.data.shape[1])
 
+    def _operator64(self, dev):
+        """fp64 device copies of A and y, built from the host arrays that are resident for the fp32 route and rebuilt
+        when new data is fed."""
+        src = (getattr(self.A, '_resident_src', None), getattr(self.y, '_resident_src', None))
+        if self._src64 is None or self._src64[0] is not src[0] or self._src64[1] is not src[1]:
+            self._A64 = self._y64 = None                 # release the old copy before the new one is made
+            self._A64 = torch.as_tensor(np.ascontiguousarray(src[0])).to(dev).to(torch.float64)
+            self._y64 = torch.as_tensor(np.ascontiguousarray(src[1])).to(dev).to(torch.float64).reshape(-1)
+            self._src64 = src
+        return self._A64, self._y64
+
+    def _step64(self, opt, count, eps, seed, offset):
+        A, _ = self.A.tensor(), self.y.tensor()          # keep the fp32 residents (and their _resident_src) current
+        dev = A.device
+        M, n = (int(s) for s in A.shape)
+        A64, y64 = self._operator64(dev)
+        lib = _lib.load()
+        cfg = _lib.LinopConfig(M, M, n, int(count), int(seed), int(offset), 0)
+        if self._key64 != (M, n, int(count)):
+            self._wsb = int(lib.hb_linop_f64_workspace_bytes(C.byref(cfg)))
+            self._ws = torch.empty(self._wsb, dtype=torch.uint8, device=dev)
+            self._zbar64 = torch.empty(int(count) * n + 4, dtype=torch.float64, device=dev)
+            self._out4 = torch.zeros(4, dtype=torch.float64, device=dev)
+            self._key64 = (M, n, int(count))
+        npar = int(lib.hb_linop_param_count(C.byref(cfg)))
+        self._pull64(opt, npar, dev)
+        e = None
+        if eps is not None:
+            e = torch.as_tensor(np.asarray(eps), dtype=torch.float64) if not isinstance(eps, torch.Tensor) else eps
+            e = e.to(dev, torch.float64).reshape(count, n).contiguous()
+        check(lib.hb_linop_elbo_local_f64(C.byref(cfg), ptr(A64), ptr(y64), ptr(self._p64), ptr(e), ptr(self._zbar64),
+                                          ptr(self._ws), self._wsb, stream()), "hb_linop_elbo_local_f64")
+        check(lib.hb_increment_i32(ptr(opt._step), stream()), "hb_increment_i32")
+        o = opt.optimizer
+        adam = _lib.AdamConfig(float(o.learning_rate), float(o.beta1), float(o.beta2), float(o.epsilon), -1.0,
+                               C.c_void_p(opt._step.data_ptr()), 0)
+        check(lib.hb_linop_elbo_update_f64(C.byref(cfg), ptr(self._p64), ptr(self._zbar64), None, ptr(self._m64), ptr(self._v64),
+                                           C.byref(adam), ptr(self._out4), ptr(self._ws), self._wsb, stream()),
+              "hb_linop_elbo_update_f64")
+        self._push64(opt, npar)
+        return self._out4[0]
+
     def step(self, opt, count, eps, seed, offset, world):
+        if self.f64 and world == 1:
+            return self._step64(opt, count, eps, seed, offset)
         A, y = self.A.tensor(), self.y.tensor()
         if self._st is None or self._st.S != count:
             st = LinearOperatorStep.__new__(LinearOperatorStep)

@@ -482,6 +482,24 @@ int hb_linop_elbo_update(const hb_linop_config* cfg, float* params, const float*
                          float lr, float b1, float b2, float eps_adam, const int* step_dev, int step_host, float* out4,
                          void* ws, size_t ws_bytes, void* stream);
 
+/* ---- the same model in float64 (csrc/linop64.cu) -------------------------------------------------------------------------
+ * The reference's float_type = float64 (henbunrc:7) for config 5: the two calls above with every pointer double, the same
+ * hb_linop_config (presplit must be 0; M > 0), the same packing and hb_linop_param_count.  zbar_stats is [S*n + 4] doubles,
+ * all-reduced (sum) by the ranks between the two calls; both calls take the SAME workspace of
+ * hb_linop_f64_workspace_bytes(cfg) (0 for an invalid cfg).
+ *   local : eps [S,n] or NULL (the library's Philox stream at (seed, offset), the fp32 draw widened to double, so both
+ *           routes see the same samples; offset a multiple of 4).  Both operator products run on hb_gemm_f64.
+ *   update: grads NULL -> no gradient stored; otherwise d ELBO_mean / d params (lower triangle of q_sqrt only).  m, v NULL ->
+ *           gradient only; otherwise TF-1 Adam by *adam (hb_adam_config: grad_scale = -1 minimises -ELBO, step counter
+ *           from step_dev when non-NULL) in the same pass that forms the q_sqrt gradient, which is never materialised; the
+ *           strict upper triangle of q_sqrt, m and v is never touched.  out4 = {ELBO, loglik, kl, 0}.
+ * Every reduction has a fixed order: results are bitwise repeatable. */
+size_t hb_linop_f64_workspace_bytes(const hb_linop_config* cfg);
+int hb_linop_elbo_local_f64(const hb_linop_config* cfg, const double* A, const double* y, const double* params,
+                            const double* eps, double* zbar_stats, void* ws, size_t ws_bytes, void* stream);
+int hb_linop_elbo_update_f64(const hb_linop_config* cfg, double* params, const double* zbar_stats, double* grads, double* m,
+                             double* v, const hb_adam_config* adam, double* out4, void* ws, size_t ws_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
