@@ -104,6 +104,7 @@ SIGNATURES = {
     "hb_density_logpdf": (_i, [_i, _c_f, _c_f, _ll, _c_f, _c_f]),
     "hb_density_logpdf_bwd": (_i, [_i, _c_f, _c_f, _ll, _c_f, _ll, _c_f, _c_f, _sz, _c_f]),
     "hb_gather_rows": (_i, [_c_f, _c_f, _c_f, _ll, _ll, _c_f]),
+    "hb_gather_rows_f64": (_i, [_c_f, _c_f, _c_f, _ll, _ll, _c_f]),
     "hb_random_index": (_i, [_c_f, _ll, _c_f, _ll, _ull, _ull, _c_f]),
     "hb_gauss_loglik_fwd": (_i, [_c_f, _c_f, _c_f, _ll, _ll, _c_f, _fl, _c_f, _c_f, _c_f, _sz, _c_f]),
     "hb_rbf_gram_fwd": (_i, [_c_f, _c_f, _i, _i, _i, _i, _c_f, _i, _c_f, _ll, _ll, _fl, _i, _i, _c_f]),
@@ -145,6 +146,9 @@ SIGNATURES = {
     "hb_amortised_param_count": (_sz, [C.POINTER(AmortisedConfig)]),
     "hb_amortised_workspace_bytes": (_sz, [C.POINTER(AmortisedConfig)]),
     "hb_amortised_elbo_step": (_i, [C.POINTER(AmortisedConfig), _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _sz, _c_f]),
+    "hb_amortised_f64_workspace_bytes": (_sz, [C.POINTER(AmortisedConfig)]),
+    "hb_amortised_elbo_step_f64": (_i, [C.POINTER(AmortisedConfig), _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, C.POINTER(AdamConfig),
+                                        _c_f, _sz, _c_f]),
     "hb_gp_small_max_n": (_i, [_i]),
     "hb_gp_small_workspace_bytes": (_sz, [C.POINTER(GpConfig), _i]),
     "hb_gp_small_step": (_i, [C.POINTER(GpConfig), _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, _c_f, C.POINTER(AdamConfig), _c_f, _sz,

@@ -9,6 +9,7 @@
 // pass that writes dELBO/dx_rec (the [S B, 784] log-density tensor is never materialised), activation-backward fused with
 // the bias-gradient column sums, tall dW reductions by deterministic split-K.
 #include "../../include/henbun_b200.h"
+#include "amortised.cuh"
 #include "gemm.cuh"
 #include "kernels.cuh"
 
@@ -69,27 +70,6 @@ Layout layout(const hb_amortised_config& c) {
   return L;
 }
 
-bool valid(const hb_amortised_config& c) {
-  if (c.B <= 0 || c.S <= 0 || c.latent <= 0) return false;
-  if (c.n_enc < 1 || c.n_enc > HB_MAX_LAYERS || c.n_dec < 1 || c.n_dec > HB_MAX_LAYERS) return false;
-  if (c.enc_nodes[c.n_enc] != 2 * c.latent || c.dec_nodes[0] != c.latent) return false;
-  if (c.dec_nodes[c.n_dec] != c.enc_nodes[0]) return false;          // gaussian(X, dec(z), var): same width as the data
-  for (int i = 0; i <= c.n_enc; ++i) if (c.enc_nodes[i] <= 0) return false;
-  for (int i = 0; i <= c.n_dec; ++i) if (c.dec_nodes[i] <= 0) return false;
-  for (int i = 0; i + 1 < c.n_enc; ++i) if (c.enc_act[i] < 0 || c.enc_act[i] > 3) return false;
-  for (int i = 0; i + 1 < c.n_dec; ++i) if (c.dec_act[i] < 0 || c.dec_act[i] > 3) return false;
-  return true;
-}
-
-size_t net_params(const int* nodes, int n, size_t start, size_t* w_off, size_t* b_off) {
-  size_t o = start;
-  for (int l = 0; l < n; ++l) {
-    w_off[l] = o; o += (size_t)nodes[l] * nodes[l + 1];
-    b_off[l] = o; o += (size_t)nodes[l + 1];
-  }
-  return o;
-}
-
 // y[rows, out] = act(x[rows, in] W + b)
 int layer_fwd(const float* x, const float* W, const float* b, float* y, int rows, int in, int out, int act, void* ws, size_t wsb,
               cudaStream_t st) {
@@ -120,6 +100,28 @@ int layer_bwd(const float* gy, const float* y, const float* x, const float* W, f
 }
 
 }  // namespace
+
+bool amortised_valid(const hb_amortised_config& c) {
+  if (c.B <= 0 || c.S <= 0 || c.latent <= 0) return false;
+  if (c.n_enc < 1 || c.n_enc > HB_MAX_LAYERS || c.n_dec < 1 || c.n_dec > HB_MAX_LAYERS) return false;
+  if (c.enc_nodes[c.n_enc] != 2 * c.latent || c.dec_nodes[0] != c.latent) return false;
+  if (c.dec_nodes[c.n_dec] != c.enc_nodes[0]) return false;          // gaussian(X, dec(z), var): same width as the data
+  for (int i = 0; i <= c.n_enc; ++i) if (c.enc_nodes[i] <= 0) return false;
+  for (int i = 0; i <= c.n_dec; ++i) if (c.dec_nodes[i] <= 0) return false;
+  for (int i = 0; i + 1 < c.n_enc; ++i) if (c.enc_act[i] < 0 || c.enc_act[i] > 3) return false;
+  for (int i = 0; i + 1 < c.n_dec; ++i) if (c.dec_act[i] < 0 || c.dec_act[i] > 3) return false;
+  return true;
+}
+
+size_t amortised_net_params(const int* nodes, int n, size_t start, size_t* w_off, size_t* b_off) {
+  size_t o = start;
+  for (int l = 0; l < n; ++l) {
+    w_off[l] = o; o += (size_t)nodes[l] * nodes[l + 1];
+    b_off[l] = o; o += (size_t)nodes[l + 1];
+  }
+  return o;
+}
+
 }  // namespace hb
 
 using namespace hb;
@@ -127,15 +129,15 @@ using namespace hb;
 extern "C" {
 
 size_t hb_amortised_param_count(const hb_amortised_config* c) {
-  if (!c || !valid(*c)) return 0;
+  if (!c || !amortised_valid(*c)) return 0;
   size_t w[HB_MAX_LAYERS], b[HB_MAX_LAYERS];
-  size_t o = net_params(c->enc_nodes, c->n_enc, 0, w, b);
-  o = net_params(c->dec_nodes, c->n_dec, o, w, b);
+  size_t o = amortised_net_params(c->enc_nodes, c->n_enc, 0, w, b);
+  o = amortised_net_params(c->dec_nodes, c->n_dec, o, w, b);
   return o + 1;
 }
 
 size_t hb_amortised_workspace_bytes(const hb_amortised_config* c) {
-  if (!c || !valid(*c)) return 0;
+  if (!c || !amortised_valid(*c)) return 0;
   return layout(*c).total + 256;
 }
 
@@ -144,7 +146,7 @@ int hb_amortised_elbo_step(const hb_amortised_config* cfg, const float* X, const
   if (!cfg || !X || !params || !grads || !out4) return HB_ERR_ARG;
   OptScope scope(cfg->opt);
   const hb_amortised_config c = *cfg;
-  if (!valid(c)) return HB_ERR_ARG;
+  if (!amortised_valid(c)) return HB_ERR_ARG;
   if (!eps && (c.offset & 3ull)) return HB_ERR_ARG;
   const Layout L = layout(c);
   if (!ws || ws_bytes < L.total + 256) return HB_ERR_WORKSPACE;
@@ -152,8 +154,8 @@ int hb_amortised_elbo_step(const hb_amortised_config* cfg, const float* X, const
   char* base = reinterpret_cast<char*>((reinterpret_cast<uintptr_t>(ws) + 255) & ~uintptr_t(255));
   auto F = [&](size_t off) { return reinterpret_cast<float*>(base + off); };
   size_t ew[HB_MAX_LAYERS], eb[HB_MAX_LAYERS], dw[HB_MAX_LAYERS], db[HB_MAX_LAYERS];
-  size_t o = net_params(c.enc_nodes, c.n_enc, 0, ew, eb);
-  o = net_params(c.dec_nodes, c.n_dec, o, dw, db);
+  size_t o = amortised_net_params(c.enc_nodes, c.n_enc, 0, ew, eb);
+  o = amortised_net_params(c.dec_nodes, c.n_dec, o, dw, db);
   const size_t var_off = o;
   float* sc = F(L.sc);
   float* out3 = sc + 8;

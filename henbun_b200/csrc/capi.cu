@@ -412,6 +412,11 @@ int hb_gather_rows(float* dst, const float* src, const long long* index, long lo
   return gather_rows(dst, src, index, n_index, row_elems, S(stream));
 }
 
+int hb_gather_rows_f64(double* dst, const double* src, const long long* index, long long n_index, long long row_elems,
+                       void* stream) {
+  return gather_rows_f64(dst, src, index, n_index, row_elems, S(stream));
+}
+
 int hb_random_index(long long* out, long long n_index, const long long* pool, long long pool_size, unsigned long long seed,
                     unsigned long long offset, void* stream) {
   return random_index(out, n_index, pool, pool_size, seed, offset, S(stream));

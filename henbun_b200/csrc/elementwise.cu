@@ -216,7 +216,8 @@ __global__ void adam_tf1_kernel(float* theta, const float* __restrict__ grad, fl
 __global__ void increment_kernel(int* p) { *p += 1; }
 
 // dst[i, :] = src[index[i], :]  (MinibatchData.get_feed_dict, Henbun/param.py:733-739, on device)
-__global__ void gather_rows_kernel(float* __restrict__ dst, const float* __restrict__ src,
+template <typename T>
+__global__ void gather_rows_kernel(T* __restrict__ dst, const T* __restrict__ src,
                                    const long long* __restrict__ index, long long n_index, long long row) {
   const long long total = n_index * row;
   for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
@@ -371,14 +372,22 @@ int adam_tf1(float* theta, const float* grad, float* m, float* v, long long n, f
   HB_CHECK_LAUNCH();
   return HB_OK;
 }
-int gather_rows(float* dst, const float* src, const long long* index, long long n_index, long long row_elems,
-                cudaStream_t st) {
+template <typename T>
+int gather_rows_t(T* dst, const T* src, const long long* index, long long n_index, long long row_elems, cudaStream_t st) {
   if (n_index < 0 || row_elems < 0) return HB_ERR_ARG;
   if (n_index * row_elems == 0) return HB_OK;
   if (!dst || !src || !index) return HB_ERR_ARG;
-  gather_rows_kernel<<<grid_for(n_index * row_elems, 256), 256, 0, st>>>(dst, src, index, n_index, row_elems);
+  gather_rows_kernel<T><<<grid_for(n_index * row_elems, 256), 256, 0, st>>>(dst, src, index, n_index, row_elems);
   HB_CHECK_LAUNCH();
   return HB_OK;
+}
+int gather_rows(float* dst, const float* src, const long long* index, long long n_index, long long row_elems,
+                cudaStream_t st) {
+  return gather_rows_t(dst, src, index, n_index, row_elems, st);
+}
+int gather_rows_f64(double* dst, const double* src, const long long* index, long long n_index, long long row_elems,
+                    cudaStream_t st) {
+  return gather_rows_t(dst, src, index, n_index, row_elems, st);
 }
 int increment_i32(int* p, cudaStream_t st) {
   increment_kernel<<<1, 1, 0, st>>>(p);

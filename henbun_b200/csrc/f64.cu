@@ -34,9 +34,24 @@ struct G64 {
   double alpha, beta;
   double* part;        // split-K partial tiles [splits][M][N] (nullptr: one split)
   int kchunk;          // k range per split (multiple of BK)
+  // epilogue and split policy of gemm64_ex (zero for every other caller): C = act(alpha op(A) op(B) + beta C + bias)
+  const double* bias;  // [N] or nullptr
+  int act;             // ACT_* (gemm.cuh)
+  int split_tall;      // split long K over CTAs up to kTallSplitCtas even when the output has many tiles
 };
 
 constexpr int BK = 16;
+constexpr int kTallSplitCtas = 592;                      // about four resident 64 x 64 CTAs per SM
+
+__device__ __forceinline__ double epilogue64(const G64& p, int c, double v) {
+  if (p.bias) v += p.bias[c];
+  switch (p.act) {
+    case ACT_SIGMOID: return 1.0 / (1.0 + exp(-v));
+    case ACT_RELU: return v > 0.0 ? v : 0.0;
+    case ACT_TANH: return tanh(v);
+    default: return v;
+  }
+}
 
 __device__ __forceinline__ bool keep_a(int tri, int m, int k) {
   switch (tri) {
@@ -202,7 +217,8 @@ __global__ void __launch_bounds__(Tile<BM, BN, WM, WN>::NT) gemm_f64_kernel(cons
           p.part[((long long)blockIdx.z * p.M + r) * p.N + c] = acc[i][j][q];
         } else if (!(p.c_tri && c > r)) {
           double* cp = p.C + (long long)r * p.ldc + c;
-          *cp = p.alpha * acc[i][j][q] + (p.beta != 0.0 ? p.beta * *cp : 0.0);
+          const double v = p.alpha * acc[i][j][q] + (p.beta != 0.0 ? p.beta * *cp : 0.0);
+          *cp = (p.bias || p.act) ? epilogue64(p, c, v) : v;
         }
       }
 }
@@ -216,8 +232,18 @@ __global__ void splitk_reduce_f64_kernel(const G64 p, int splits) {
     double s = 0.0;
     for (int z = 0; z < splits; ++z) s += p.part[(long long)z * total + e];
     double* cp = p.C + (long long)r * p.ldc + c;
-    *cp = p.alpha * s + (p.beta != 0.0 ? p.beta * *cp : 0.0);
+    const double v = p.alpha * s + (p.beta != 0.0 ? p.beta * *cp : 0.0);
+    *cp = (p.bias || p.act) ? epilogue64(p, c, v) : v;
   }
+}
+
+// K splits wanted for `tiles` output tiles and a k range of klen, before the workspace bound: small outputs with long K
+// spread K over about two waves of CTAs; split_tall (tall reductions such as dW = x^T dz over S B rows) up to about four
+// CTAs per SM whatever the output size
+int wanted_splits(long long tiles, int klen, int split_tall) {
+  const long long target = split_tall ? kTallSplitCtas : 296;
+  if (tiles >= (split_tall ? target : 74) || klen < 1024) return 1;
+  return (int)std::min<long long>(std::min(32, klen / 256), (target + tiles - 1) / tiles);
 }
 
 template <int BM, int BN, int WM, int WN>
@@ -229,9 +255,8 @@ int launch_gemm_f64(G64 p, void* ws, size_t ws_bytes, cudaStream_t st) {
   tile_k_range(q, 0, BM, 0, BN, kb, ke);
   const int klen = ke - kb;
   int splits = 1;
-  const long long tiles = (long long)gx * gy;
-  if (ws && tiles < 74 && klen >= 1024) {                // small output, long K: spread K over about two waves of CTAs
-    splits = (int)std::min<long long>(std::min(32, klen / 256), (296 + tiles - 1) / tiles);
+  if (ws) {
+    splits = wanted_splits((long long)gx * gy, klen, p.split_tall);
     while (splits > 1 && (size_t)splits * p.M * p.N * sizeof(double) > ws_bytes) --splits;
   }
   if (splits > 1) {
@@ -256,6 +281,17 @@ int gemm_f64(const G64& p0, void* ws, size_t ws_bytes, cudaStream_t st) {
   if (p.M <= 16) return launch_gemm_f64<16, 64, 16, 16>(p, ws, ws_bytes, st);
   return launch_gemm_f64<64, 64, 32, 32>(p, ws, ws_bytes, st);
 }
+
+}  // namespace
+
+size_t gemm64_split_bytes(int M, int N, int K, int split_tall) {
+  if (M <= 0 || N <= 0 || K <= 0) return 0;
+  const long long tiles = (long long)cdiv(N, 64) * cdiv(M, M <= 16 ? 16 : 64);
+  const int s = wanted_splits(tiles, K, split_tall);
+  return s > 1 ? (size_t)s * M * N * sizeof(double) : 0;
+}
+
+namespace {
 
 int check_g64(const G64& p) {
   if (p.M < 0 || p.N < 0 || p.K < 0) return HB_ERR_ARG;
@@ -400,6 +436,12 @@ inline int split64(int w) { return ((cdiv(w, NB64) + 1) / 2) * NB64; }
 int gemm64(const Ctx64& c, const double* A, long long lda, int transA, int a_tri, const double* B, long long ldb, int transB,
            int b_tri, double* C, long long ldc, int c_tri, int M, int N, int K, double alpha, double beta) {
   G64 p{A, lda, transA, a_tri, B, ldb, transB, b_tri, C, ldc, c_tri, M, N, K, alpha, beta, nullptr, 0};
+  return gemm_f64(p, c.ws, c.ws_bytes, c.st);
+}
+
+int gemm64_ex(const Ctx64& c, const double* A, long long lda, int transA, const double* B, long long ldb, int transB, double* C,
+              long long ldc, int M, int N, int K, double beta, const double* bias, int act, int split_tall) {
+  G64 p{A, lda, transA, 0, B, ldb, transB, 0, C, ldc, 0, M, N, K, 1.0, beta, nullptr, 0, bias, act, split_tall};
   return gemm_f64(p, c.ws, c.ws_bytes, c.st);
 }
 

@@ -24,6 +24,12 @@ struct Ctx64 {
 int ensure_attrs64();
 int gemm64(const Ctx64& c, const double* A, long long lda, int transA, int a_tri, const double* B, long long ldb, int transB,
            int b_tri, double* C, long long ldc, int c_tri, int M, int N, int K, double alpha, double beta);
+// C = act(op(A) op(B) + beta C + bias) without triangular masks (bias [N] or nullptr, act ACT_* of gemm.cuh).  split_tall:
+// split a long K over CTAs even when the output has many tiles (tall reductions), in a fixed split order.  The bytes of
+// partial tiles it may use: gemm64_split_bytes.
+int gemm64_ex(const Ctx64& c, const double* A, long long lda, int transA, const double* B, long long ldb, int transB, double* C,
+              long long ldc, int M, int N, int K, double beta, const double* bias, int act, int split_tall);
+size_t gemm64_split_bytes(int M, int N, int K, int split_tall);
 int potrf_cols64(const Ctx64& c, double* A, long long lda, int c0, int w, int n);
 int chol_rev_cols64(const Ctx64& c, const double* L, long long ldl, double* G, long long ldg, int c0, int w, int n);
 

@@ -74,6 +74,8 @@ int transform_logjac_bwd(int kind, const float* x, long long total, float p0, fl
                          cudaStream_t st);
 int gather_rows(float* dst, const float* src, const long long* index, long long n_index, long long row_elems,
                 cudaStream_t st);
+int gather_rows_f64(double* dst, const double* src, const long long* index, long long n_index, long long row_elems,
+                    cudaStream_t st);
 
 // ---- UnitRBF Gram (gram.cu) ----
 int rbf_gram_fwd(const float* X, const float* X2, int n, int n2, int D, long long sX, long long sX2,

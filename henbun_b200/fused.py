@@ -694,15 +694,20 @@ class LinopElboBinding(_Float64Masters):
         return st.out4[0]
 
 
-class AmortisedElboBinding(object):
+class AmortisedElboBinding(_Float64Masters):
     """BASELINE config 4 recognised in a traced objective:
         self.q_local = self.enc(self.X);  x_rec = self.dec(self.q_local)
         ELBO = reduce_sum(gaussian(self.X, x_rec, self.var)) - self.KL(graph_key.LOCAL)
     with enc / dec = nn.NeuralNet, q_local = LOCAL variationals.Normal([latent]) (diagonal), X = MinibatchData.
     One call of hb_amortised_elbo_step (csrc/amortised.cu) on the gathered minibatch writes every gradient into the
-    Optimizer's flat buffer, laid out as [enc w0 | enc b0 | ... | dec w0 | dec b0 | ... | var]."""
+    Optimizer's flat buffer, laid out as [enc w0 | enc b0 | ... | dec w0 | dec b0 | ... | var].
+    Under float_type = float64 (henbunrc:7) with one process (`f64`, fixed when compile() binds), the step, TF-1 Adam
+    included, is hb_amortised_elbo_step_f64 (csrc/amortised64.cu) on fp64 master copies (_Float64Masters) and on this
+    step's rows gathered from a resident fp64 copy of the data."""
 
-    def __init__(self, model, X, enc, dec, q, var):
+    _grad64 = False                     # the fp64 step keeps its gradient in its workspace
+
+    def __init__(self, model, X, enc, dec, q, var, f64=False):
         self.model, self.X, self.enc, self.dec, self.q, self.var = model, X, enc, dec, q, var
         g = object.__getattribute__
         order = []
@@ -710,6 +715,8 @@ class AmortisedElboBinding(object):
             for layer in net._matbias_list:
                 order += [g(layer, 'w'), g(layer, 'b')]
         self.var_order = order + [var]
+        self.f64 = bool(f64)
+        self.fused_adam = self.f64
         self.lib = _lib.load()
         self._key = None
 
@@ -758,20 +765,19 @@ class AmortisedElboBinding(object):
             return None
         if _variationals_of(model) != [q]:
             return None
-        return AmortisedElboBinding(model, X, enc, dec, q, var)
+        from ._settings import settings
+        f64 = str(settings.dtypes.float_type) == 'float64' and parallel.world()[0] == 1
+        return AmortisedElboBinding(model, X, enc, dec, q, var, f64=f64)
 
     def per_sample(self):
         return int(self.X.tensor().shape[0]) * int(self.q._shape[0])
 
-    def step(self, opt, count, eps, seed, offset):
+    def _config(self, B, count, f64):
         from .nn import _act_name
-        X = self.X.tensor()
-        B = int(X.shape[0])
-        lat = int(self.q._shape[0])
-        key = (B, count)
+        key = (B, count, f64)
         if self._key != key:
             cfg = _lib.AmortisedConfig()
-            cfg.B, cfg.S, cfg.latent = B, int(count), lat
+            cfg.B, cfg.S, cfg.latent = B, int(count), int(self.q._shape[0])
             for name, net in (('enc', self.enc), ('dec', self.dec)):
                 setattr(cfg, 'n_' + name, len(net._matbias_list))
                 nodes = getattr(cfg, name + '_nodes'); acts = getattr(cfg, name + '_act')
@@ -780,18 +786,66 @@ class AmortisedElboBinding(object):
                 for i, a in enumerate(net.neuron_types):
                     acts[i] = _lib.ACT[_act_name(a)]
             self._cfg = cfg
-            self._wsb = int(self.lib.hb_amortised_workspace_bytes(C.byref(cfg)))
+            size = self.lib.hb_amortised_f64_workspace_bytes if f64 else self.lib.hb_amortised_workspace_bytes
+            self._wsb = int(size(C.byref(cfg)))
             if self._wsb == 0:
                 raise _lib.HenbunB200Error("hb_amortised_elbo_step rejected the network shapes")
-            self._ws = torch.empty(self._wsb, dtype=torch.uint8, device=X.device)
-            self._out4 = torch.zeros(4, device=X.device)
+            dev = self.X.tensor().device
+            self._ws = None                              # release the old workspace before the new one is made
+            self._ws = torch.empty(self._wsb, dtype=torch.uint8, device=dev)
+            self._out4 = torch.zeros(4, device=dev, dtype=torch.float64 if f64 else torch.float32)
             self._key = key
-        cfg = self._cfg
+        return self._cfg
+
+    def _eps(self, eps, count, B, dev, dtype):
+        if eps is None:
+            return None
+        e = torch.as_tensor(np.asarray(eps), dtype=dtype) if not isinstance(eps, torch.Tensor) else eps
+        return e.to(dev, dtype).reshape(count, B, int(self.q._shape[0])).contiguous()
+
+    def _minibatch64(self, dev):
+        """This step's rows (the index the fp32 route gathered) from an fp64 device copy of X.data, rebuilt when the data
+        is replaced."""
+        src = self.X.data
+        if self._src64 is not src:
+            self._X64 = None                             # release the old copy before the new one is made
+            self._X64 = torch.as_tensor(np.ascontiguousarray(src, dtype=np.float64)).to(dev)
+            self._src64 = src
+        idx = self.X.last_index.to(device=dev, dtype=torch.int64).contiguous()
+        row = int(self._X64.shape[1])
+        out = torch.empty((idx.numel(), row), dtype=torch.float64, device=dev)
+        check(self.lib.hb_gather_rows_f64(ptr(out), ptr(self._X64), ptr(idx), idx.numel(), row, stream()), "hb_gather_rows_f64")
+        return out
+
+    def _step64(self, opt, count, eps, seed, offset):
+        dev = self.X.tensor().device
+        X64 = self._minibatch64(dev)
+        B = int(X64.shape[0])
+        cfg = self._config(B, int(count), True)
         cfg.seed, cfg.offset = int(seed), int(offset)
-        e = None
-        if eps is not None:
-            e = torch.as_tensor(np.asarray(eps), dtype=torch.float32) if not isinstance(eps, torch.Tensor) else eps
-            e = e.to(X.device, torch.float32).reshape(count, B, lat).contiguous()
+        npar = int(self.lib.hb_amortised_param_count(C.byref(cfg)))
+        self._pull64(opt, npar, dev)
+        check(self.lib.hb_increment_i32(ptr(opt._step), stream()), "hb_increment_i32")
+        o = opt.optimizer
+        adam = _lib.AdamConfig(float(o.learning_rate), float(o.beta1), float(o.beta2), float(o.epsilon), -1.0,
+                               C.c_void_p(opt._step.data_ptr()), 0)
+        e = self._eps(eps, count, B, dev, torch.float64)
+        check(self.lib.hb_amortised_elbo_step_f64(C.byref(cfg), ptr(X64), ptr(self._p64), ptr(e), None, ptr(self._out4),
+                                                  ptr(self._m64), ptr(self._v64), C.byref(adam), ptr(self._ws), self._wsb,
+                                                  stream()), "hb_amortised_elbo_step_f64")
+        self._push64(opt, npar)
+        return self._out4[0]
+
+    def step(self, opt, count, eps, seed, offset, world=None):
+        """Called with `world` (fused_adam: the float64 route) the step applies Adam itself; without it the fp32 step
+        writes the gradient into opt._flat_grad and the caller applies Adam."""
+        if world is not None:
+            return self._step64(opt, count, eps, seed, offset)
+        X = self.X.tensor()
+        B = int(X.shape[0])
+        cfg = self._config(B, int(count), False)
+        cfg.seed, cfg.offset = int(seed), int(offset)
+        e = self._eps(eps, count, B, X.device, torch.float32)
         check(self.lib.hb_amortised_elbo_step(C.byref(cfg), ptr(X), ptr(opt._flat), ptr(e), ptr(opt._flat_grad), ptr(self._out4),
                                               ptr(self._ws), self._wsb, stream()), "hb_amortised_elbo_step")
         return self._out4[0]

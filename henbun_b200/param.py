@@ -525,6 +525,7 @@ class MinibatchData(Data):
         if self._resident is None:
             self._resident = torch.as_tensor(np.ascontiguousarray(self.data)).to(self._dtype).to(_device())
         idx = index if isinstance(index, torch.Tensor) else torch.as_tensor(np.asarray(index, dtype=np.int64))
+        self.last_index = idx               # the rows of this feed, for a binding that gathers its own copy of the data
         if self._dtype == torch.float32:
             self._tensor = ops.gather_rows(self._resident, idx.to(self._resident.device))
         else:

@@ -176,6 +176,9 @@ int hb_density_logpdf_bwd(int kind, const float* const* args, const long long* p
 /* MinibatchData.get_feed_dict (param.py:733-739) on device: dst[i,:] = src[index[i],:], index int64. */
 int hb_gather_rows(float* dst, const float* src, const long long* index, long long n_index, long long row_elems,
                    void* stream);
+/* The same in double (the float64 route of the amortised model gathers its minibatch from a resident fp64 copy). */
+int hb_gather_rows_f64(double* dst, const double* src, const long long* index, long long n_index, long long row_elems,
+                       void* stream);
 /* Indexer.train_index (model.py:147-149) on device: out[i] = pool[j_i], j_i uniform in [0, pool_size) with replacement,
  * drawn from Philox(seed, offset) (two 32-bit words per index; 2 * ceil(n_index / 2) stream positions).  pool == NULL:
  * out[i] = j_i.  Feeds hb_gather_rows without any host work or host->device copy per step. */
@@ -450,6 +453,17 @@ size_t hb_amortised_param_count(const hb_amortised_config* cfg);
 size_t hb_amortised_workspace_bytes(const hb_amortised_config* cfg);
 int hb_amortised_elbo_step(const hb_amortised_config* cfg, const float* X, const float* params, const float* eps, float* grads,
                            float* out4, void* ws, size_t ws_bytes, void* stream);
+/* The reference's float_type = float64 (henbunrc:7) for config 4 (csrc/amortised64.cu): the step above with every pointer
+ * double, the same hb_amortised_config, packing, hb_amortised_param_count and out4, and a workspace of
+ * hb_amortised_f64_workspace_bytes(cfg) (0 for an invalid cfg).  eps [S, B, latent] or NULL: the library's Philox stream at
+ * (seed, offset), the fp32 draw widened to double at the same stream positions, so both routes see the same samples (offset
+ * a multiple of 4).  adam_m / adam_v NULL -> gradient only, into grads; otherwise TF-1 Adam by *adam on params after the
+ * gradient (grads may then be NULL).  Every product runs on hb_gemm_f64's DMMA kernel; every reduction has a fixed order
+ * and none uses atomics, so results are bitwise repeatable. */
+size_t hb_amortised_f64_workspace_bytes(const hb_amortised_config* cfg);
+int hb_amortised_elbo_step_f64(const hb_amortised_config* cfg, const double* X, double* params, const double* eps, double* grads,
+                               double* out4, double* adam_m, double* adam_v, const hb_adam_config* adam, void* ws,
+                               size_t ws_bytes, void* stream);
 
 /* ---- fused ELBO + gradient + Adam of the linear-operator model (BASELINE config 5) ---------------------
  * q = variationals.Normal([n], q_shape='fullrank') (variationals.py:94-96,144-146,185-186,225-230) observed through a
